@@ -26,6 +26,9 @@ Outside the timed regions the same line also carries (every block degrades to {"
 the same four shapes with the same method (value kernel-only, e2e from pinned host buffers), as replicas on every rank;
 when the reference cannot be imported it falls back to the torch-CPU BF16-emulated GEMM (oracle port) on a bounded sample.
 Its `cpu_baseline` block is that CPU port in both cases (the reference has no CPU implementation of this path).
+
+`--dump-outputs DIR` (dense workload) writes D of the four shapes as the last timed step left them, as float32 .npy files
+(see `dump_outputs`). The inputs come from fixed seeds, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -323,6 +326,27 @@ def time_dense_step(args, world, device, probs, gemm, on_first_call=None):
     return per_shape_ms, per_step_ms, clocks.summary(), wall
 
 
+DUMP_LIMIT_BYTES = 64_000_000      # all files together, .npy headers included
+NPY_HEADER_BYTES = 4096            # an upper bound of the header np.save writes for a 2-D array
+
+
+def dump_outputs(out_dir, probs):
+    """D of every dense problem to `out_dir`/d_<M>x<N>x<K>.npy in float32 (BF16 widens exactly). Smallest first, each file
+    gets an equal share of what is left of 64 MB, so small outputs are written whole and what they leave goes to the larger
+    ones; a D larger than its share keeps the rows of a sorted sample drawn with a fixed seed, the same rows in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_LIMIT_BYTES
+    for i, p in enumerate(sorted(probs, key=lambda p_: p_['d'].numel())):
+        d = p['d'].float().cpu()
+        rows = (left // (len(probs) - i) - NPY_HEADER_BYTES) // (d.shape[1] * d.element_size())
+        if rows < d.shape[0]:
+            d = d[torch.randperm(d.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values]
+        path = os.path.join(out_dir, f"d_{p['m']}x{p['n']}x{p['k']}.npy")
+        np.save(path, d.numpy())
+        left -= os.path.getsize(path)
+
+
 def dense_ab_block(probs, dg, iters=20):
     """Per dense shape: ours vs the unmodified reference kernel, same tensors, same flush + CUDA-event method, interleaved."""
     try:
@@ -384,6 +408,8 @@ def run_dense(args, rank, world, device):
     launches0 = _lib.launch_count()
     per_shape_ms, per_step_ms, clock_summary, t_wall = time_dense_step(args, world, device, probs, dg.fp8_gemm_nt, note_tile)
     retimed = RETIMED
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, probs)
     launches = (_lib.launch_count() - launches0) * args.steps // (args.steps + args.warmup)
     step_ms = allreduce_max(sum(per_shape_ms), world, device)
     flops = sum(2.0 * p['m'] * p['n'] * p['k'] for p in probs)
@@ -1119,7 +1145,12 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='dense workload: skip the reference A/B, grouped and EP blocks')
     ap.add_argument('--extras-timeout', type=float, default=420.0)
+    ap.add_argument('--dump-outputs', metavar='DIR', help='dense workload: write what the last timed step computed to DIR')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.workload != 'dense' or args.impl != 'ours'):
+        ap.error('--dump-outputs covers the dense workload of --impl ours')
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get('RANK', '0'))

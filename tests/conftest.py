@@ -13,4 +13,5 @@ def pytest_configure(config):
 @pytest.fixture(scope='session')
 def cpu_golden():
     import torch
-    return torch.load(os.path.join(os.path.dirname(__file__), 'golden', 'cpu_golden.pt'), weights_only=False)
+    from golden import store
+    return store.load(os.path.join(os.path.dirname(__file__), 'golden'), 'cpu_golden')

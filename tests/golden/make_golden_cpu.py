@@ -6,7 +6,7 @@ Sources executed (unmodified, imported from the reference install oracle/_ref wh
   * deep_gemm/testing/numeric.py:5-11 calc_diff
   * tests/test_layout.py:20-42        get_mn_major_tma_aligned_packed_ue8m0_tensor_torch_impl -- the reference's own
                                       bit-exact statement of the packed-UE8M0 wire format (loaded by path)
-Output: tests/golden/cpu_golden.pt
+Output: tests/golden/cpu_golden.*.pt (tests/golden/store.py)
 """
 import importlib.util
 import os
@@ -78,9 +78,9 @@ def main():
         out['calc_diff'].append({'x': a, 'y': a + 0.01 * b_, 'd': float(calc_diff(a, a + 0.01 * b_))})
     out['calc_diff'].append({'x': torch.zeros(4), 'y': torch.zeros(4), 'd': float(calc_diff(torch.zeros(4), torch.zeros(4)))})
 
-    path = os.path.join(HERE, 'cpu_golden.pt')
-    torch.save(out, path)
-    print('wrote', path, os.path.getsize(path), 'bytes')
+    import store
+    for path in store.save(out, HERE, 'cpu_golden'):
+        print('wrote', path, os.path.getsize(path), 'bytes')
 
 
 if __name__ == '__main__':

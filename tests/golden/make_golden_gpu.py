@@ -3,7 +3,7 @@ reference install oracle/_ref built by oracle/build_ref.sh; nothing here touches
 
 For a few small seeded problems it stores the FP8 operands, scale factors and the output of the unmodified
 reference (`deep_gemm.fp8_gemm_nt`, `m_grouped_fp8_gemm_nt_masked`, `m_grouped_fp8_gemm_nt_contiguous`).
-Output: gpurun_out/gpu_golden.pt (copy to tests/golden/gpu_golden.pt and commit).
+Output: tests/golden/gpu_golden.*.pt (tests/golden/store.py), or under the directory given as the first argument.
 """
 import os
 import random
@@ -128,10 +128,11 @@ def main():
                                  'c': c.cpu(), 'd': d.cpu(), 'ks': ks, 'gran_k': gran_k, 'k_alignment': k_alignment})
     ref.set_mk_alignment_for_contiguous_layout(128)
 
-    os.makedirs(os.path.join(REPO, 'gpurun_out'), exist_ok=True)
-    path = os.path.join(REPO, 'gpurun_out', 'gpu_golden.pt')
-    torch.save(out, path)
-    print('wrote', path, os.path.getsize(path))
+    import store
+    out_dir = sys.argv[1] if len(sys.argv) > 1 else HERE
+    os.makedirs(out_dir, exist_ok=True)
+    for path in store.save(out, out_dir, 'gpu_golden'):
+        print('wrote', path, os.path.getsize(path))
 
 
 if __name__ == '__main__':

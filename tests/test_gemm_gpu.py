@@ -1,6 +1,6 @@
 """GPU parity tests (run with `-m gpu` on a B200). Everything goes through the public API -> C ABI -> CUDA kernels and
 is checked against the CPU oracle (oracle/blockwise.py) on seeded inputs, against committed golden fixtures produced
-by the reference's own SM100 kernel (tests/golden/gpu_golden.pt), and -- at BASELINE.json's full sizes -- through
+by the reference's own SM100 kernel (tests/golden/gpu_golden.*.pt), and -- at BASELINE.json's full sizes -- through
 size-independent properties (linearity in the power-of-two scales, row/column permutation equivariance, zero rows).
 
 Tolerance: every e4m3 x e4m3 product and every UE8M0 scale is exact, so the only freedom versus the oracle is the
@@ -497,12 +497,10 @@ def test_full_size_dense_properties(dg):
 
 
 def test_golden_outputs_of_the_reference_kernel(dg):
-    """tests/golden/gpu_golden.pt holds outputs of the reference's own SM100 kernel (generated on a B200 by
+    """tests/golden/gpu_golden.*.pt hold outputs of the reference's own SM100 kernel (generated on a B200 by
     tests/golden/make_golden_gpu.py). Same FP8 inputs + scale factors -> the outputs must match bit for bit."""
-    path = os.path.join(HERE, 'golden', 'gpu_golden.pt')
-    if not os.path.exists(path):
-        pytest.skip('gpu_golden.pt not generated yet')
-    golden = torch.load(path, weights_only=False)
+    from golden import store
+    golden = store.load(os.path.join(HERE, 'golden'), 'gpu_golden')
     for case in golden['dense']:
         qa = (case['a'].cuda().view(torch.float8_e4m3fn), case['sfa'].cuda())
         qb = (case['b'].cuda().view(torch.float8_e4m3fn), case['sfb'].cuda())

@@ -52,7 +52,10 @@ def test_version_and_knobs_roundtrip(lib):
     dg.set_num_sms(147)
     assert lib.lib().dgb200_get_num_sms() == 147
     dg.set_num_sms(0)
-    assert lib.lib().dgb200_get_num_sms() == 0
+    # 0 reads back as 0 until the library has set up a device (the GPU tests before this one do in a whole-suite run),
+    # from then on as that device's SM count
+    n = lib.lib().dgb200_get_num_sms()
+    assert n == 0 or n == torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
     with pytest.raises(RuntimeError):
         dg.set_num_sms(-2)
     with pytest.raises(RuntimeError):
@@ -269,3 +272,32 @@ def test_tools_and_bench_compile():
     assert len(files) > 10
     for f in files:
         compile(open(f).read(), f, 'exec')
+
+
+def test_bench_dump_outputs_stays_within_64_mb_and_samples_the_same_rows(tmp_path):
+    """bench.py --dump-outputs: float32 files, 64 MB in all at the benchmark's shapes; the small outputs are whole, the
+    largest keeps a sorted, seeded sample of as many rows as the rest of the budget holds, so two runs write identical files."""
+    import numpy as np
+
+    import bench
+    probs = [dict(m=m, n=n, k=k, d=torch.randn((m, n), generator=torch.Generator().manual_seed(m)).to(torch.bfloat16))
+             for m, n, k in bench.DENSE_SHAPES]
+    for run in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / run), probs)
+    total = sum(f.stat().st_size for f in (tmp_path / 'a').iterdir())
+    assert 60_000_000 < total <= 64_000_000
+    sampled = 0
+    for p in probs:
+        name = f"d_{p['m']}x{p['n']}x{p['k']}.npy"
+        got = np.load(tmp_path / 'a' / name)
+        assert got.dtype == np.float32 and got.shape[1] == p['n']
+        assert np.array_equal(got, np.load(tmp_path / 'b' / name))
+        full = p['d'].float().numpy()
+        if got.shape[0] == p['m']:
+            assert np.array_equal(got, full)
+            continue
+        sampled += 1
+        row_of = {full[i].tobytes(): i for i in range(p['m'])}
+        picked = [row_of[r.tobytes()] for r in got]
+        assert picked == sorted(set(picked))
+    assert sampled == 1

@@ -146,8 +146,8 @@ def test_grouped_oracles_agree_with_per_group_dense():
 # ------------------------------------------------------------------------------------------------ oracle vs the reference KERNEL
 def _gpu_golden():
     import os
-    path = os.path.join(os.path.dirname(__file__), 'golden', 'gpu_golden.pt')
-    return torch.load(path, weights_only=False)
+    from golden import store
+    return store.load(os.path.join(os.path.dirname(__file__), 'golden'), 'gpu_golden')
 
 
 def _assert_oracle_close(got, ref_out, what):
@@ -167,7 +167,7 @@ def _assert_oracle_close(got, ref_out, what):
 
 
 def test_oracle_reproduces_the_reference_kernels_golden_outputs():
-    """Direct pin of the CPU restatement on the outputs of the UNMODIFIED reference kernel (tests/golden/gpu_golden.pt,
+    """Direct pin of the CPU restatement on the outputs of the UNMODIFIED reference kernel (tests/golden/gpu_golden.*.pt,
     made on a B200 by tests/golden/make_golden_gpu.py): dense (+ C accumulation, BF16 and FP32), masked, contiguous
     (+ psum), MN-major (tn) and the K-grouped weight gradient."""
     g = _gpu_golden()
@@ -206,3 +206,11 @@ def test_oracle_reproduces_the_reference_kernels_golden_outputs():
         got = oracle.k_grouped_fp8_gemm_tn_contiguous((f8(case['a']), case['sfa']), (f8(case['b']), case['sfb']), case['c'], case['ks'],
                                                       gran_k=case['gran_k'])
         _assert_oracle_close(got, case['d'], case['name'])
+
+
+def test_golden_fixture_files_stay_within_1_mb():
+    import os
+    from golden import store
+    golden = os.path.join(os.path.dirname(__file__), 'golden')
+    sizes = {f: os.path.getsize(os.path.join(golden, f)) for f in os.listdir(golden) if os.path.isfile(os.path.join(golden, f))}
+    assert max(sizes.values()) <= store.PART_LIMIT, sizes
